@@ -26,17 +26,25 @@ One JSON line is printed by rank 0:
                same mix of rays (rays_per_sample is printed by both)
 
 Workloads (BASELINE.json configs): soup = configs[1] (default; --tris 10000000 / 50000000 for the scenes
-beyond L2), killeroo = configs[2] (scenes/killeroo-simple.pbrt at 1920x1080x256, staged by
-__graft_entry__.build() into baseline/_scenes/), instanced = configs[3].
+beyond L2), killeroo = configs[2] (the reference's scenes/killeroo-simple.pbrt at 1920x1080x256, stored in
+tests/golden/killeroo/), instanced = configs[3].
+
+--dump-outputs DIR writes what the timed path returned in its last timed step: film.npy, the merged film (H x W x 4
+float32: RGB sums and filter-weight sum per pixel; above 64 MB a fixed, seeded sample of pixels with their indices in
+film_pixel_index.npy), and ray_counts.npy (camera, regular, shadow ray tests of rank 0; float64).  The inputs depend only on
+the arguments, so two builds can be compared output for output.  Nothing is written into the tree: run-time files go
+to a temporary directory.
 """
 import argparse
 import ctypes as C
 import json
+import lzma
 import math
 import os
 import re
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -98,7 +106,22 @@ class ClockSampler:
                 "samples": len(self.samples)}
 
 
-SCENES_DIR = os.path.join(ROOT, "baseline", "_scenes")   # staged by __graft_entry__.build(); git-ignored, travels with gpurun
+KILLEROO_DIR = os.path.join(ROOT, "tests", "golden", "killeroo")   # the scene file and its mesh (xz-compressed)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def stage_killeroo(dst, text=None):
+    """Writes killeroo-simple.pbrt (or `text` in its place) and the geometry/killeroo.pbrt it includes under `dst`;
+    returns the scene file's path."""
+    os.makedirs(os.path.join(dst, "geometry"), exist_ok=True)
+    with lzma.open(os.path.join(KILLEROO_DIR, "killeroo.pbrt.xz")) as f, open(os.path.join(dst, "geometry", "killeroo.pbrt"), "wb") as g:
+        g.write(f.read())
+    if text is None:
+        text = open(os.path.join(KILLEROO_DIR, "killeroo-simple.pbrt")).read()
+    path = os.path.join(dst, "killeroo-simple.pbrt")
+    with open(path, "w") as f:
+        f.write(text)
+    return path
 
 
 def build_scene(args):
@@ -108,21 +131,14 @@ def build_scene(args):
         return pb.HostScene.instanced_soup(args.tris, grid=args.grid, xres=args.xres, yres=args.yres, spp=args.spp, maxdepth=args.maxdepth)
     if args.workload == "killeroo":
         # BASELINE.json configs[2]: the reference's own scenes/killeroo-simple.pbrt, only film size and sample count changed
-        src = os.path.join(SCENES_DIR, "killeroo-simple.pbrt")
-        if not os.path.exists(src):
-            raise SystemExit("bench.py --workload killeroo: %s is missing (run __graft_entry__.build() where /root/reference exists)" % src)
-        text = open(src).read()
+        text = open(os.path.join(KILLEROO_DIR, "killeroo-simple.pbrt")).read()
         text, n1 = re.subn(r'"integer xresolution" \[\d+\] "integer yresolution" \[\d+\]',
                            '"integer xresolution" [%d] "integer yresolution" [%d]' % (args.xres, args.yres), text, count=1)
         text, n2 = re.subn(r'"integer pixelsamples" \[\d+\]', '"integer pixelsamples" [%d]' % args.spp, text, count=1)
         text, n3 = re.subn(r'Integrator "path"', 'Integrator "path" "integer maxdepth" [%d]' % args.maxdepth, text, count=1)
         assert n1 == 1 and n2 == 1 and n3 == 1
-        dst = os.path.join(SCENES_DIR, "killeroo-%dx%dx%d.pbrt" % (args.xres, args.yres, args.spp))   # next to geometry/ (Include is relative)
-        if int(os.environ.get("RANK", "0")) == 0 or not os.path.exists(dst):
-            tmp = dst + ".%d.tmp" % os.getpid()
-            open(tmp, "w").write(text)
-            os.replace(tmp, dst)
-        return pb.HostScene.from_file(dst)
+        with tempfile.TemporaryDirectory(prefix="pb2_bench_") as tmp:   # the parser reads the Include while loading
+            return pb.HostScene.from_file(stage_killeroo(tmp, text))
     return pb.HostScene.soup(args.tris, seed=args.seed, jitter=args.jitter, xres=args.xres, yres=args.yres,
                              spp=args.spp, maxdepth=args.maxdepth)
 
@@ -232,6 +248,23 @@ def workload_config(args, parallelism):
                         "next to the scene (node records + leaf records = %.0f MB); no explicit flush" % scene_mb)
 
 
+def dump_outputs(directory, film, stats):
+    """film.npy (whole, or above DUMP_LIMIT_BYTES a seeded sample of pixels whose flat indices go to
+    film_pixel_index.npy) and ray_counts.npy; see the module docstring."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    film = np.ascontiguousarray(film, np.float32)
+    if film.nbytes > DUMP_LIMIT_BYTES:
+        pixels = film.reshape(-1, film.shape[-1])
+        keep = DUMP_LIMIT_BYTES // 2 // pixels[0].nbytes
+        index = np.sort(np.random.default_rng(0).choice(len(pixels), keep, replace=False))
+        film = pixels[index]
+        np.save(os.path.join(directory, "film_pixel_index.npy"), index.astype(np.float64))
+    np.save(os.path.join(directory, "film.npy"), film)
+    np.save(os.path.join(directory, "ray_counts.npy"),
+            np.array([stats.camera_rays, stats.regular_rays, stats.shadow_rays], np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -251,7 +284,12 @@ def main():
     ap.add_argument("--maxdepth", type=int, default=None)
     ap.add_argument("--ref-seconds", type=float, default=15.0, help="CPU seconds per reference sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the film and ray counts of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    sys.dont_write_bytecode = True   # the tree may be read-only; nothing is cached there
     inst, kill = args.workload == "instanced", args.workload == "killeroo"
     if args.tris is None: args.tris = 100000 if inst else WORKLOAD["tris"]
     if args.spp is None: args.spp = 128 if inst else 256 if kill else WORKLOAD["spp"]
@@ -335,6 +373,8 @@ def main():
     node_visits, prim_tests, rays_frame, launches = (int(x) for x in counts.tolist())
     ms_per_step = ms_total / args.steps
     value = n_samples / ms_per_step / 1e3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, film.cpu().numpy(), s)   # the film and stats of the last timed step
 
     # end to end through the host-buffer ABI call pb2_render_path, at every N: structs in, this rank's tiles rendered, the
     # NCCL reduce inside the call, and the merged film copied into rank 0's page-locked host buffer inside the call

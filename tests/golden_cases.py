@@ -227,3 +227,34 @@ def bsdf_frames(n, seed):
     dpdu[::4] += 0.2 * ns[::4]
     wo, wi = unit(rs.normal(size=(n, 3))), unit(rs.normal(size=(n, 3)))
     return np.ascontiguousarray(np.concatenate([nrm, ns, dpdu, wo, wi, rs.uniform(0, 1, (n, 2))], 1), np.float32)
+
+
+def digest(a):
+    """sha256 of an array's bytes: what tests/golden/reference_digests.json stores where the test asks for every bit."""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+LIGHT_STRATEGIES = ("spatial", "uniform")
+
+
+def light_strategy_scene_text(scenes_dir, strategy):
+    """tests/scenes/lights.pbrt with another "lightsamplestrategy" than its "power"."""
+    import os
+    text = open(os.path.join(scenes_dir, "lights.pbrt")).read()
+    return text.replace('"string lightsamplestrategy" "power"', '"string lightsamplestrategy" "%s"' % strategy)
+
+
+PYRAMID_CASES = [(1, 1, 1, 0), (1, 7, 3, 0), (5, 1, 1, 2), (13, 31, 3, 1), (16, 4, 1, 0), (33, 64, 3, 2), (100, 3, 1, 1)]   # w, h, channels, wrap
+
+
+def pyramid_textures(pb):
+    """Random images of awkward sizes (1 x N, N x 1, primes, already a power of two) as pb2_textures: (case, texture, texels);
+    the texels array must outlive the texture."""
+    import ctypes as C
+    rs = np.random.RandomState(9)
+    for (w, h, ch, wrap) in PYRAMID_CASES:
+        texels = rs.uniform(0, 2, (h, w, ch)).astype(np.float32)
+        t = pb.Texture(channels=ch, width=w, height=h, wrap=wrap, do_trilinear=0, max_anisotropy=8.0, su=1, sv=1, du=0, dv=0,
+                       texels=texels.ctypes.data_as(C.POINTER(C.c_float)))
+        yield "%dx%dx%d_wrap%d" % (w, h, ch, wrap), t, texels

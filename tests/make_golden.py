@@ -149,6 +149,33 @@ def record_env_distribution(ref):
     print("env distribution", nu, nv)
 
 
+def record_reference_digests(ref):
+    """sha256 digests (tests/golden_cases.py digest) of reference outputs that tests compare bit for bit: the light
+    distribution, Li samples, image and ray counts of tests/scenes/lights.pbrt under the other two light-sampling strategies,
+    MIPMap::pyramid of random images of awkward sizes, and the Sobol tables (SobolMatrices32, VdCSobolMatrices /
+    VdCSobolMatricesInv for every resolution from 2 to 2^25 pixels)."""
+    import json
+    out = {}
+    for strategy in gc.LIGHT_STRATEGIES:
+        hs = pb.HostScene.from_string(gc.light_strategy_scene_text(os.path.join(ROOT, "tests", "scenes"), strategy))
+        rs = ref.scene(hs)
+        pix, sn = gc.sample_ids(hs.film.contents.full_resolution[0], hs.film.contents.full_resolution[1],
+                                hs.params.contents.samples_per_pixel, 3000, 13)
+        li, _ = rs.li_samples(pix, sn)
+        img, _, st = rs.render(n_threads=0)
+        out["lights_" + strategy] = dict(light_distribution=gc.digest(rs.light_distribution(gc.points_for(hs.nodes(), 400, 15))),
+                                         li=gc.digest(li), image=gc.digest(img),
+                                         rays=[int(st.camera_rays), int(st.regular_rays), int(st.shadow_rays)])
+    out["pyramids"] = {case: [[list(lv.shape), gc.digest(lv)] for lv in ref.texture_pyramid(t)] for case, t, _ in gc.pyramid_textures(pb)}
+    _, mats = ref.sobol_tables(1)
+    out["sobol_matrices32"] = gc.digest(mats)
+    out["vdc_sobol"] = {str(m): gc.digest(ref.sobol_tables(m)[0]) for m in range(1, 26)}
+    with open(os.path.join(OUT, "reference_digests.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("reference digests:", ", ".join(sorted(out)))
+
+
 def main():
     ref = pyoracle.reference()
     if ref is None:
@@ -180,6 +207,7 @@ def main():
     record_textures(ref)
     record_filters(ref)
     record_hlbvh(ref)
+    record_reference_digests(ref)
     # the metal material's default eta / k: copper's measured spectra through Spectrum::FromSampled (metal.cpp:121-126)
     eta, k = ref.copper_rgb()
     np.savez_compressed(os.path.join(OUT, "metal_defaults.npz"), eta=eta, k=k)

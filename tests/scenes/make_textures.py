@@ -1,5 +1,6 @@
-"""Writes the small image files the textured golden scenes read (tests/scenes/textures/).  Deterministic; the files are
-committed, this script documents how they were made:
+"""Writes the small image files the textured golden scenes read (tests/scenes/textures/), and the OpenEXR reader's
+fixtures written by the OpenEXR library (tests/golden/openexr/).  Deterministic; the files are committed, this script
+documents how they were made:
 
     python tests/scenes/make_textures.py
 """
@@ -10,6 +11,7 @@ import zlib
 import numpy as np
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "textures")
+OUT_OPENEXR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "golden", "openexr")
 
 
 def write_pfm(path, img):
@@ -128,6 +130,42 @@ def write_exr(path, img, compression="zip"):
         f.write(header + table + b"".join(chunks))
 
 
+def write_exr_openexr(path, img, compression):
+    """The same picture written by the OpenEXR library itself (as bundled with OpenCV), for the codecs write_exr does not
+    implement and for ZIP / ZIPS as the library compresses them: half B / G / R channels, RLE (1 line per block), ZIPS (1),
+    ZIP (16), PIZ (32) or B44 (lossy; the reader must refuse it)."""
+    os.environ["OPENCV_IO_ENABLE_OPENEXR"] = "1"
+    import cv2
+    comp = {"rle": 1, "zips": 2, "zip": 3, "piz": 4, "b44": 6}[compression]
+    bgr = np.ascontiguousarray(np.asarray(img, np.float32)[:, :, ::-1])
+    assert cv2.imwrite(path, bgr, [cv2.IMWRITE_EXR_TYPE, cv2.IMWRITE_EXR_TYPE_HALF, cv2.IMWRITE_EXR_COMPRESSION, comp])
+
+
+def with_decreasing_line_order(src, dst):
+    """The scan-line file `src` laid out as lineOrder DECREASING_Y: the same blocks stored from the last to the first, the
+    offset table still indexed from the first block."""
+    data = open(src, "rb").read()
+    pos, order_at = 8, None
+    while data[pos] != 0:                                   # attributes: name \0 type \0 size data
+        name_end = data.index(b"\0", pos)
+        type_end = data.index(b"\0", name_end + 1)
+        size = struct.unpack_from("<i", data, type_end + 1)[0]
+        if data[pos:name_end] == b"lineOrder":
+            order_at = type_end + 5
+        pos = type_end + 5 + size
+    table = pos + 1
+    n = (struct.unpack_from("<Q", data, table)[0] - table) // 8
+    offsets = list(struct.unpack_from("<%dQ" % n, data, table)) + [len(data)]
+    blocks = [data[offsets[i]:offsets[i + 1]] for i in range(n)]
+    header = bytearray(data[:table])
+    header[order_at] = 1
+    new, at = [0] * n, table + 8 * n
+    for i in reversed(range(n)):
+        new[i], at = at, at + len(blocks[i])
+    with open(dst, "wb") as f:
+        f.write(bytes(header) + struct.pack("<%dQ" % n, *new) + b"".join(blocks[::-1]))
+
+
 def pattern(w, h, seed):
     """coloured tiles with a smooth gradient on top: detail at the texel scale and below"""
     rs = np.random.RandomState(seed)
@@ -163,6 +201,14 @@ def main():
     write_exr(os.path.join(OUT, "tiles_24x18_zips.exr"), hdr, "zips")
     write_exr(os.path.join(OUT, "tiles_24x18_none.exr"), hdr, "none")
     np.savez_compressed(os.path.join(OUT, "decoded_8bit.npz"), png=rgb8, tga=rgb8b, exr=hdr.astype(np.float32))
+    # 70 lines: two full PIZ blocks of 32 and a short one
+    hdr2 = (pattern(40, 70, 7) * np.float32(3.0)).astype(np.float16)
+    hdr2[5, 9] = [2000.0, 0.0004, 0.0]
+    os.makedirs(OUT_OPENEXR, exist_ok=True)
+    for codec in ("rle", "zips", "zip", "piz", "b44"):
+        write_exr_openexr(os.path.join(OUT_OPENEXR, "tiles_40x70_%s.exr" % codec), hdr2, codec)
+    with_decreasing_line_order(os.path.join(OUT_OPENEXR, "tiles_40x70_piz.exr"), os.path.join(OUT_OPENEXR, "tiles_40x70_piz_decreasing.exr"))
+    np.savez_compressed(os.path.join(OUT_OPENEXR, "decoded.npz"), exr=hdr2.astype(np.float32))
 
 
 if __name__ == "__main__":

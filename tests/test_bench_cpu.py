@@ -24,6 +24,27 @@ def test_reference_arm_prints_the_contract_line():
     assert d["gpu_launches"] == 0
 
 
+def test_dump_of_a_film_beyond_the_limit_is_a_seeded_sample(tmp_path):
+    """--dump-outputs stays within 64 MB: a larger film is written as a fixed sample of its pixels plus their indices."""
+    import numpy as np
+
+    import bench
+    from pbrt_v3_b200 import Stats
+    h, w = 2400, 2000                                            # 76.8 MB of rgbw
+    film = np.arange(h * w * 4, dtype=np.float32).reshape(h, w, 4)
+    st = Stats(camera_rays=h * w, regular_rays=7, shadow_rays=3)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), film, st)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["film.npy", "film_pixel_index.npy", "ray_counts.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    sample, index = np.load(tmp_path / "a" / "film.npy"), np.load(tmp_path / "a" / "film_pixel_index.npy")
+    assert sample.dtype == np.float32 and index.dtype == np.float64 and len(sample) == len(index) > 1000000
+    assert (np.diff(index) > 0).all() and np.array_equal(sample, film.reshape(-1, 4)[index.astype(np.int64)])
+    assert np.array_equal(index, np.load(tmp_path / "b" / "film_pixel_index.npy"))
+    assert np.load(tmp_path / "a" / "ray_counts.npy").tolist() == [h * w, 7, 3]
+
+
 def test_reference_arm_under_torchrun_prints_once():
     """Launched like the driver launches N > 1: rank 0 alone runs the reference and prints; the other ranks exit 0."""
     import socket

@@ -812,9 +812,9 @@ def test_texture_combinators(pb):
 def test_openexr_reader(pb, tmp_path):
     """ReadImage for OpenEXR scan-line files (imageio.cpp:125-151 reads them through OpenEXR's RgbaInputFile): half channels
     stored B, G, R; ZIP blocks of 16 lines (the last one short) with the byte-delta predictor and the even / odd byte split,
-    blocks stored raw when they do not shrink, uncompressed files, and the PIZ codec - the committed files of tests/scenes/make_textures.py,
-    the container this library writes itself, and (where the reference's bundled OpenEXR sources are present) OpenEXR's own
-    test images, which hold one picture under every codec."""
+    blocks stored raw when they do not shrink, uncompressed files, and the RLE and PIZ codecs - the committed files of
+    tests/scenes/make_textures.py (those under tests/golden/openexr/ written by the OpenEXR library itself) and the container
+    this library writes itself."""
     tex = os.path.join(SCENES, "textures")
     want = np.load(os.path.join(tex, "decoded_8bit.npz"))["exr"]
     for kind in ("zip", "zips", "none"):
@@ -830,16 +830,16 @@ def test_openexr_reader(pb, tmp_path):
                                   'Material "matte" "texture Kd" "t"\nShape "sphere"\nWorldEnd\n' % tex)
     t = hs.desc.contents.textures[0]
     assert np.array_equal(np.ctypeslib.as_array(t.texels, shape=(18, 24, 3)), want[::-1])
-    ilm = "/root/reference/src/ext/openexr/OpenEXR/IlmImfTest"
-    if os.path.exists(os.path.join(ilm, "comp_none.exr")):
-        base = pb.read_image(os.path.join(ilm, "comp_none.exr"))
-        assert base.shape == (675, 587, 3) and np.isfinite(base).all()
-        for codec in ("rle", "zips", "zip", "piz"):      # piz: value table + wavelet + Huffman with run lengths
-            assert np.array_equal(pb.read_image(os.path.join(ilm, "comp_%s.exr" % codec)).view(np.uint32), base.view(np.uint32)), codec
-        up, down = (pb.read_image(os.path.join(ilm, "lineOrder_%s.exr" % o)) for o in ("increasing", "decreasing"))   # PIZ, 119 lines
-        assert up.shape == (119, 237, 3) and np.array_equal(up.view(np.uint32), down.view(np.uint32))
-        # the lossy codecs are reported, not misread
-        before = pb.lib().pb2h_error_count()
-        with pytest.raises(RuntimeError):
-            pb.read_image(os.path.join(ilm, "comp_b44.exr"))
-        assert pb.lib().pb2h_error_count() > before
+    # files written by the OpenEXR library itself (tests/golden/openexr/, made by tests/scenes/make_textures.py), one picture
+    # under every lossless codec: PIZ (value table + wavelet + Huffman with run lengths) in blocks of 32 lines, the last one
+    # short, also stored in decreasing line order
+    ilm = os.path.join(GOLDEN, "openexr")
+    want = np.load(os.path.join(ilm, "decoded.npz"))["exr"]
+    for codec in ("rle", "zips", "zip", "piz", "piz_decreasing"):
+        got = pb.read_image(os.path.join(ilm, "tiles_40x70_%s.exr" % codec))
+        assert got.shape == (70, 40, 3) and np.array_equal(got.view(np.uint32), want.view(np.uint32)), codec
+    # the lossy codecs are reported, not misread
+    before = pb.lib().pb2h_error_count()
+    with pytest.raises(RuntimeError):
+        pb.read_image(os.path.join(ilm, "tiles_40x70_b44.exr"))
+    assert pb.lib().pb2h_error_count() > before

@@ -1,8 +1,9 @@
 """The CPU oracle (oracle/pb2_oracle.cpp) against (a) golden vectors recorded from the unmodified reference
 (tests/make_golden.py), (b) the reference's own known-answer tests for this path (src/tests/shapes.cpp,
-src/tests/sampling.cpp), and (c) where it exists, the compiled reference itself (oracle/_ref), live.
+src/tests/sampling.cpp), and (c) digests of further reference results (tests/golden/reference_digests.json).
 Everything here runs on the CPU; bit-exact unless said otherwise.
 """
+import json
 import os
 
 import numpy as np
@@ -12,6 +13,11 @@ import golden_cases as gc
 from conftest import GOLDEN, SCENES
 
 SCENE_CASES = ["soup", "killeroo_like", "materials", "instances", "specular", "substrate", "metal", "uber", "roughglass", "lights", "params"]
+
+
+def reference_digests():
+    with open(os.path.join(GOLDEN, "reference_digests.json")) as f:
+        return json.load(f)
 
 
 def load_scene(pb, name):
@@ -64,9 +70,10 @@ def test_port_matches_reference_golden(pb, port, name):
 
 
 @pytest.mark.parametrize("name", SCENE_CASES)
-def test_port_matches_compiled_reference_live(pb, port, reference, name):
-    hs = load_scene(pb, name)
-    a, b = recompute(pb, reference, hs), recompute(pb, port, hs)
+def test_port_matches_compiled_reference_live(pb, port, name):
+    """Byte for byte what the compiled reference computed for the scene (recorded by tests/make_golden.py)."""
+    a = np.load(os.path.join(GOLDEN, name + ".npz"))
+    b = recompute(pb, port, load_scene(pb, name))
     for k in ("hits", "occluded", "halton", "light_distribution", "li", "pfilm", "image", "rays"):
         assert a[k].tobytes() == b[k].tobytes(), k
 
@@ -81,21 +88,23 @@ def test_port_filters_match_reference_golden(pb, port, case):
     assert [st.camera_rays, st.regular_rays, st.shadow_rays] == [int(x) for x in g["rays_" + case]]
 
 
-@pytest.mark.parametrize("strategy", ["spatial", "uniform"])
-def test_port_delta_lights_other_strategies_live(pb, port, reference, strategy):
-    text = open(os.path.join(SCENES, "lights.pbrt")).read().replace('"string lightsamplestrategy" "power"', '"string lightsamplestrategy" "%s"' % strategy)
-    hs = pb.HostScene.from_string(text)
-    a, b = recompute(pb, reference, hs), recompute(pb, port, hs)
-    for k in ("light_distribution", "li", "image", "rays"):
-        assert a[k].tobytes() == b[k].tobytes(), k
+@pytest.mark.parametrize("strategy", gc.LIGHT_STRATEGIES)
+def test_port_delta_lights_other_strategies_live(pb, port, strategy):
+    """The compiled reference's results for tests/scenes/lights.pbrt under another light-sampling strategy, as digests."""
+    want = reference_digests()["lights_" + strategy]
+    b = recompute(pb, port, pb.HostScene.from_string(gc.light_strategy_scene_text(SCENES, strategy)))
+    for k in ("light_distribution", "li", "image"):
+        assert gc.digest(b[k]) == want[k], k
+    assert b["rays"].tolist() == want["rays"]
 
 
-def test_port_filters_match_compiled_reference_live(pb, port, reference):
+def test_port_filters_match_compiled_reference_live(pb, port):
+    """Byte for byte the compiled reference's image for every filter case (recorded by tests/make_golden.py)."""
+    g = np.load(os.path.join(GOLDEN, "filters.npz"))
     for case in sorted(gc.FILTER_CASES):
         hs = pb.HostScene.from_string(gc.filter_scene_text(SCENES, case))
-        a, _, _ = reference.scene(hs).render(n_threads=1)
         b, _, _ = port.scene(hs).render(n_threads=1)
-        assert a.tobytes() == b.tobytes(), case
+        assert g["image_" + case].tobytes() == b.tobytes(), case
 
 
 @pytest.mark.parametrize("case", sorted(gc.ANALYTIC_SCENES))
@@ -286,21 +295,18 @@ def test_empty_and_degenerate_inputs(pb, port):
     assert h["prim"][0] >= 0 and h["prim"][1] == -1 and h["prim"][2] == -1
 
 
-def test_killeroo_simple_fingerprint_of_the_surveyed_reference(pb, reference, tmp_path):
+def test_killeroo_simple_fingerprint_of_the_surveyed_reference(pb, port, tmp_path):
     """SURVEY.md section 9: `pbrt --outfile k8.pfm scenes/killeroo-simple.pbrt` of the reference binary gives md5
-    5424ce0f17db0c040e0f988ebcfe4b4d with 16 870 506 regular + 6 157 124 shadow ray tests.  The same file parsed by
-    THIS repo's host front end (parser, loop subdivision, transforms, SAH BVH builder), rendered by oracle/_ref (the
-    reference's own sources behind ref_harness.cpp) and written by our PFM writer must give those bytes: one test pins
-    the harness, the parser, the subdivision and the builder to the surveyed binary."""
+    5424ce0f17db0c040e0f988ebcfe4b4d with 16 870 506 regular + 6 157 124 shadow ray tests.  The same file (stored in
+    tests/golden/killeroo/) parsed by THIS repo's host front end (parser, loop subdivision, transforms, SAH BVH builder),
+    rendered by the port and written by our PFM writer must give those bytes: one test pins the port, the parser, the
+    subdivision and the builder to the surveyed binary."""
     import hashlib
-    from conftest import ROOT
-    scene = os.path.join(ROOT, "baseline", "_scenes", "killeroo-simple.pbrt")
-    if not os.path.exists(scene):
-        pytest.skip("baseline/_scenes/killeroo-simple.pbrt not staged (no /root/reference at build time)")
-    hs = pb.HostScene.from_file(scene)
+    from bench import stage_killeroo
+    hs = pb.HostScene.from_file(stage_killeroo(str(tmp_path)))
     d = hs.desc.contents
     assert d.n_prims == 66533 and d.n_nodes == 59188 + 59189
-    img, _, st = reference.scene(hs).render(n_threads=0)
+    img, _, st = port.scene(hs).render(n_threads=0)
     assert img.shape == (700, 700, 3)
     assert (int(st.camera_rays), int(st.regular_rays), int(st.shadow_rays)) == (3920000, 16870506, 6157124)
     out = str(tmp_path / "k8.pfm")
@@ -327,18 +333,13 @@ def test_library_texture_pyramids_are_the_reference_mipmaps(pb):
     assert resampled >= 4
 
 
-def test_library_texture_pyramids_match_reference_live(pb, reference):
-    """... and against the reference live, on random images of awkward sizes (1 x N, N x 1, primes, already a power of two)."""
-    import ctypes as C
-    rs = np.random.RandomState(9)
-    for (w, h, ch, wrap) in [(1, 1, 1, 0), (1, 7, 3, 0), (5, 1, 1, 2), (13, 31, 3, 1), (16, 4, 1, 0), (33, 64, 3, 2), (100, 3, 1, 1)]:
-        texels = rs.uniform(0, 2, (h, w, ch)).astype(np.float32)
-        t = pb.Texture(channels=ch, width=w, height=h, wrap=wrap, do_trilinear=0, max_anisotropy=8.0, su=1, sv=1, du=0, dv=0,
-                       texels=texels.ctypes.data_as(C.POINTER(C.c_float)))
-        a, b = pb.texture_pyramid(t), reference.texture_pyramid(t)
-        assert len(a) == len(b)
-        for la, lb in zip(a, b):
-            assert la.shape == lb.shape and np.array_equal(gc.bits(la), gc.bits(lb)), (w, h, ch, wrap)
+def test_library_texture_pyramids_match_reference_live(pb):
+    """... and against the reference on random images of awkward sizes (1 x N, N x 1, primes, already a power of two): shape
+    and digest of every level of the reference's pyramid."""
+    want = reference_digests()["pyramids"]
+    for case, t, _texels in gc.pyramid_textures(pb):
+        got = [[list(lv.shape), gc.digest(lv)] for lv in pb.texture_pyramid(t)]
+        assert got == want[case], case
 
 
 def test_sobol_sampler_matches_reference_golden(pb):
@@ -355,14 +356,14 @@ def test_sobol_sampler_matches_reference_golden(pb):
     assert (hdim < 2).sum() > 10 and (got[hdim < 2] < 1).all()
 
 
-def test_sobol_tables_are_the_reference_tables(pb, reference):
+def test_sobol_tables_are_the_reference_tables(pb):
     """The generator matrices (from scipy's copy of the Joe-Kuo direction numbers) equal the reference's SobolMatrices32, and
     the two SobolIntervalToIndex tables the library derives from dimensions 0 and 1 by inverting a matrix over GF(2) equal
-    VdCSobolMatrices / VdCSobolMatricesInv for every resolution from 2 to 2^25 pixels."""
+    VdCSobolMatrices / VdCSobolMatricesInv for every resolution from 2 to 2^25 pixels (digests of the reference's tables)."""
     import ctypes as C
+    want = reference_digests()
     mats = np.fromfile(os.path.join(os.path.dirname(pb.__file__), "lib", "sobol_matrices32.bin"), "<u4").reshape(1024, 52)
-    _, ref_mats = reference.sobol_tables(1)
-    assert np.array_equal(mats, ref_mats)
+    assert gc.digest(mats) == want["sobol_matrices32"]
     film = pb.FilmDesc()
     film.filter_radius[0] = film.filter_radius[1] = 0.5
     pp = pb.PathParams(samples_per_pixel=1, sampler=pb.PB2_SAMPLER_SOBOL)
@@ -371,8 +372,7 @@ def test_sobol_tables_are_the_reference_tables(pb, reference):
         film.full_resolution[0], film.full_resolution[1] = res, 1
         film.cropped_pixel_bounds[0], film.cropped_pixel_bounds[1], film.cropped_pixel_bounds[2], film.cropped_pixel_bounds[3] = 0, 0, res, 1
         _, tab = pb.sobol_samples_host(C.byref(film), C.byref(pp), np.zeros((1, 2), np.int32), np.zeros(1, np.int64), np.zeros(1, np.int32), tables=True)
-        want, _ = reference.sobol_tables(m)
-        assert np.array_equal(tab, want), m
+        assert gc.digest(tab) == want["vdc_sobol"][str(m)], m
 
 
 def test_environment_map_distribution_is_the_reference_distribution(pb):
